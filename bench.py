@@ -2,6 +2,7 @@
 """bench.py -- benchmarks of the NeRSemble render hot path on B200 (one JSON line on rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|2occ|3|4|5] [--scaling strong|weak] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default (what the driver runs): BASELINE.json config 2 -- 4096 rays x 256 samples = 2^20 samples, 32-member hash
 ensemble with full-size tables (16 levels x 2^19), T = 24, fused forward + alpha composite.
@@ -26,6 +27,12 @@ march (--disable_occupancy_grid) full gradient step on N GPUs with the gradient 
 
 `--impl reference` times the CPU oracle port of the reference's path (its GPU dependencies tiny-cuda-nn / nerfacc /
 nerfstudio are not installable here) on the host cores, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller as DIR/<name>.npy
+(float32, or float64 for integers): config 2 the render op's per-ray outputs (rgb, accumulation, depth, deformation,
+num_samples_per_ray, packed_info) and the plugin call's as e2e_<name>; configs 3 / 5 the training step's per-ray outputs
+and loss; config 4 the gathered frame (rgb) and rank 0's rows of the other outputs.  Inputs are seeded, so two builds
+run with the same arguments can be compared file for file; above 64 MB in all a fixed, seeded sample is written.
 """
 from __future__ import annotations
 
@@ -261,8 +268,10 @@ def run_reference(args):
         return
     S = synthetic_params()
     o, d, t = synthetic_rays(RAYS, 1000)
-    reps = max(1, min(args.steps, 5))
-    _, sec, threads, n = cpu_oracle(S, o[:PARITY_RAYS], d[:PARITY_RAYS], t[:PARITY_RAYS], repeats=reps)
+    reps = args.steps
+    rgb, sec, threads, n = cpu_oracle(S, o[:PARITY_RAYS], d[:PARITY_RAYS], t[:PARITY_RAYS], repeats=reps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, host_arrays({"rgb": rgb}))
     v = n / sec / 1e6
     sample = f"{PARITY_RAYS} rays x {SAMPLES_PER_RAY} samples ({n} samples) per step, full-size tables, oracle/pipeline.py torch CPU fp32; 1 warm-up + median of {reps}"
     print(json.dumps({
@@ -336,7 +345,8 @@ _GRAPHS: list = []
 
 
 def timed(D, fn, K, sampler=None):
-    """K calls of fn bracketed by barrier + synchronize on both sides; CUDA-event milliseconds (this rank)."""
+    """K calls of fn bracketed by barrier + synchronize on both sides; returns (CUDA-event milliseconds of this rank,
+    what the last call returned)."""
     import torch
     e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
     D.barrier()
@@ -344,12 +354,41 @@ def timed(D, fn, K, sampler=None):
         sampler.active = True
     e0.record()
     for _ in range(K):
-        fn()
+        last = fn()
     e1.record()
     D.barrier()
     if sampler is not None:
         sampler.active = False
-    return e0.elapsed_time(e1)
+    return e0.elapsed_time(e1), last
+
+
+DUMP_BYTES = 60 << 20             # 62.9 MB of array data: the files stay under 64 MB with their .npy headers
+
+
+def host_arrays(outputs, prefix=""):
+    """The tensors among a call's outputs (name -> tensor; other values and names starting with '_' are skipped), copied
+    to the host: float64 as it is, other floating point as float32, integers and booleans as float64 (exact)."""
+    import torch
+    arrs = {}
+    for k, v in outputs.items():
+        if torch.is_tensor(v) and not k.startswith("_"):
+            v = v.detach().cpu()
+            arrs[prefix + k] = (v.float() if v.is_floating_point() and v.dtype != torch.float64 else v.double()).numpy()
+    return arrs
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes every array as out_dir/<name>.npy, so that two builds run with the same arguments (same
+    seeded inputs) can be compared output for output.  Above DUMP_BYTES in all, every array is cut to the same fraction
+    of its elements, flattened, at positions drawn with a fixed seed (the same for every run of the same shapes)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, a.size * DUMP_BYTES // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(SEED).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def graphed(fn, dev):
@@ -447,7 +486,10 @@ def run_config2(args, occ=False):
         step_fn, was_graphed = (lambda: render(o_w, d_w, t_w)), False
     for _ in range(W):
         step_fn()
-    ms_value = timed(D, step_fn, K, sampler)
+    ms_value, last = timed(D, step_fn, K, sampler)
+    dump = {}
+    if args.dump_outputs and rank == 0:     # strong scaling replays a graph: its result is the all-gathered RGB
+        dump = host_arrays({"rgb": rgb_all} if strong else last)
     # fused field kernel alone (CUDA events around the launch, separate pass so that the events do not sit in the graph)
     for _ in range(2):
         render(o_s, d_s, t_s, time_field=False)
@@ -462,7 +504,7 @@ def run_config2(args, occ=False):
         weak_fn, _ = graphed(lambda: render(o_w, d_w, t_w), dev)
         for _ in range(W):
             weak_fn()
-        ms_weak = timed(D, weak_fn, K)
+        ms_weak, _ = timed(D, weak_fn, K)
 
     # ---- timed region 2 (e2e): the plugin call with HOST buffers ----
     n_loc = hi - lo
@@ -499,8 +541,10 @@ def run_config2(args, occ=False):
     e2e_samples.zero_()
     step_e2e(count=True)
     samples_e2e_step = int(e2e_samples.item())                  # marched by the occupancy sampler (~256 per ray)
-    ms_e2e = timed(D, step_e2e, K, sampler)
+    ms_e2e, last_e2e = timed(D, step_e2e, K, sampler)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump.update(host_arrays(last_e2e, prefix="e2e_"))
     e2e_l2 = None
     if rank == 0 and not occ:
         # the plugin path (occupancy march) and the op path (fixed march) integrate the same medium over the same span
@@ -555,6 +599,8 @@ def run_config2(args, occ=False):
             line["parity"] = parity
         if cpu is not None:
             line["cpu_baseline"] = cpu
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
         if parity is not None and not (parity["rgb_l2_max"] < 1e-3):
             sys.stderr.write(f"parity FAILED: max per-ray RGB L2 vs the oracle = {parity['rgb_l2_max']:.3e} >= 1e-3\n")
@@ -566,8 +612,11 @@ def run_config2(args, occ=False):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 20; config 4: 24, every timestep's frame once)")
     ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="2", choices=["2", "2occ", "3", "4", "5"])
     ap.add_argument("--scaling", default="auto", choices=["auto", "strong", "weak"])
@@ -579,6 +628,12 @@ def main():
     ap.add_argument("--height", type=int, default=1088)
     ap.add_argument("--width", type=int, default=1920)
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = N_TIMESTEPS if args.config == "4" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    import torch
+    torch.manual_seed(SEED)           # the training configs' sampler jitter: the same inputs on every run
     if args.impl == "reference":
         return run_reference(args)
     if args.config in ("2", "2occ"):

@@ -80,10 +80,13 @@ def _train_loop(args, D, model, opts, params, batch, rb, with_allreduce, reduce_
     n_samples = torch.zeros((), dtype=torch.long, device=D.dev)
 
     def timed_step():
-        out, _ = step(True)
+        out, loss = step(True)
         n_samples.add_(out["num_samples_per_ray"].sum())
-    ms = B.timed(D, timed_step, K, sampler)
+        return out, loss
+    ms, (last_out, last_loss) = B.timed(D, timed_step, K, sampler)
     sampler.stop_flag = True
+    if args.dump_outputs and D.rank == 0:
+        B.dump_outputs(args.dump_outputs, B.host_arrays({**last_out, "loss": last_loss}))
     for e, h in zip(marks, hmarks):
         for i, k in enumerate(phases):
             phases[k] += e[i].elapsed_time(e[i + 1]) / len(marks)
@@ -215,6 +218,7 @@ def run_config4(args):
         gather_rows_round_robin(out["rgb"], out=frame_buf, scratch=gather_buf)      # NCCL all-gather + one strided copy
         n_samples.add_(out["num_samples_per_ray"].sum())
         state["f"] += 1
+        return out
 
     with torch.no_grad():
         render_frame(); render_frame()
@@ -222,9 +226,11 @@ def run_config4(args):
         sampler = B.ClockSampler(D.local_rank)
         if rank == 0:
             sampler.start(); time.sleep(0.05)
-        K = n_frames if args.steps == 20 else args.steps      # default: all 24 timesteps once
-        ms = B.timed(D, render_frame, K, sampler)
+        K = args.steps
+        ms, last = B.timed(D, render_frame, K, sampler)
         sampler.stop_flag = True
+        if args.dump_outputs and rank == 0:     # the gathered frame, and this rank's rows of the other outputs
+            B.dump_outputs(args.dump_outputs, B.host_arrays({**last, "rgb": frame_buf}))
         # sharded vs unsharded: the last frame again on rank 0 alone (chunk boundaries differ, pixels must not)
         max_diff = None
         if rank == 0 and world > 1:
